@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/sec of the Self-Forcing hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One STEP = one generation block of the server loop (release_server.py:636-736) at
 BASELINE configs[1]: Krea-14B dims (40 layers, d=5120, ffn 13824, 40 heads), 832x480,
@@ -23,6 +23,10 @@ N > 1 : ONE video stream on all N GPUs (strong scaling; realtime_video_b200/para
         the decoder with a warm feature cache; frames/s, conv TF/s and algorithmic HBM GB/s vs the measured peak.
 --impl reference : the reference algorithm on the host CPU cores (oracle port, torch fp32, all
         threads) on a bounded sample of the same workload, scaled to frames/s.
+--dump-outputs DIR : after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32):
+        ``frames`` [1, 12, 3, 480, 832] and, for the block workload, that block's denoised ``latents``
+        [1, 3, 16, 60, 104].  Weights, prompt and noise are seeded, so two builds run with the same arguments can
+        be compared output for output.
 """
 from __future__ import annotations
 
@@ -242,6 +246,20 @@ def _claim_stdout():
         os.dup2(2, 1)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path: str, arrays: dict):
+    """Write each host tensor of ``arrays`` as ``path/<name>.npy`` in float32."""
+    import numpy as np
+    total = sum(a.numel() * 4 for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"outputs to dump take {total} bytes, over {DUMP_LIMIT_BYTES}"
+    out = Path(path)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a.to(torch.float32).numpy())
+
+
 def emit(line: dict):
     data = (json.dumps(line) + "\n").encode()
     if _JSON_FD is None:
@@ -412,6 +430,8 @@ def run_vae_workload(args, dev, rank, world, barrier, max_over_ranks):
         launches = ops.launch_count - n0
         clk = clocks.stop() if rank == 0 else None
         ms = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"frames": px.float().cpu()})
         # one profiled step (per-launch events) for the conv family's TF/s
         ops.profile_begin()
         p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -501,7 +521,13 @@ def main():
                     help="issue every DiT block as ONE C-ABI call (kr_dit_block_fwd; same launches, less host work; "
                          "single-GPU bf16 passes with a warm prompt cache)")
     ap.add_argument("--watchdog-s", type=int, default=600, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -567,9 +593,10 @@ def main():
     use_graphs = args.graphs == "on"
     transformer.model.use_block_fwd = args.block_fwd == "on"
 
-    def measure(sp: bool, steps: int, seed: int, profile_step: bool):
+    def measure(sp: bool, steps: int, seed: int, profile_step: bool, keep_outputs: bool = False):
         """W warm-up blocks, then ``steps`` timed blocks (CUDA events, barrier + synchronize on both sides, max over
-        ranks); optionally ONE more block with per-launch events for the kernel split."""
+        ranks); optionally ONE more block with per-launch events for the kernel split.  ``keep_outputs``: copy what
+        the last timed block returned to the host, as ``out["outputs"]``."""
         if sp and pp_mode:
             from realtime_video_b200.parallel import LayerPipeline
             if transformer.model.pp is None:
@@ -608,6 +635,8 @@ def main():
             out["ms"] = max_over_ranks(e0.elapsed_time(e1))
             if decode:
                 assert px.shape == (1, 12, 3, 480, 832) and px.dtype == torch.float32
+            if keep_outputs and decode and rank == 0:
+                out["outputs"] = {"frames": px.float().cpu(), "latents": sess.last_pred.float().cpu()}
             if profile_step:
                 barrier()
                 ops.profile_begin()
@@ -676,7 +705,9 @@ def main():
                 "d2h": (jpeg_bytes // max(1, steps) + 48) if jpeg else host_out.numel() * host_out.element_size()}
 
     streams = 1 if sp_mode else world           # independent video streams in flight
-    main_run = measure(sp_mode, K, 42, profile_step=True)
+    main_run = measure(sp_mode, K, 42, profile_step=True, keep_outputs=args.dump_outputs is not None)
+    if "outputs" in main_run:
+        dump_outputs(args.dump_outputs, main_run.pop("outputs"))
     e2e_run = measure_e2e(sp_mode, K, 1042)
 
     # same end-to-end loop with the byte egress kernel (SURVEY.md 8f.2): kr_frames_to_rgb8 does the reference's

@@ -2,9 +2,10 @@
 (release_server.py:344-736) on boxes where the reference checkout (and its FastAPI / omegaconf dependencies)
 does not exist: ``bench.py``, ``smoke()`` and the ``-m gpu`` tests drive the server's per-block sequence
 through it.  In a real deployment the reference's OWN ``GenerationSession`` runs unmodified on the drop-in
-classes; ``tests/test_reference_callers_cpu.py`` executes exactly that (unmodified release_server.py) and
-asserts bit-equality with this stand-in block by block, and ``tests/golden/server_loop_small.npz`` holds the
-same loop executed by the reference modules alone.
+classes; ``tests/golden/reference_callers_small.npz`` records exactly that (unmodified release_server.py, bit-equal
+with this stand-in block by block when recorded), ``tests/test_reference_callers_cpu.py`` checks this stand-in
+against the record, and ``tests/golden/server_loop_small.npz`` holds the same loop executed by the reference
+modules alone.
 
 Per block (release_server.py:636-736):
     recompute_kv_cache  -> block >= 1: re-initialise the cache, one DiT pass at t=0 over the

@@ -1,8 +1,11 @@
 """Row a1 / b of SURVEY.md §8: the reference's OWN callers, unmodified, on the drop-in classes.
 
-Each case runs tests/run_reference_callers.py in a subprocess (release_server.py flips process-wide torch state at
-import).  Needs the reference checkout (/root/reference: the build container; absent on the GPU box, where the
-bit-equal harness stand-ins are used instead — tests/test_server_loop_gpu.py, tests/test_pipeline_gpu.py)."""
+What those callers compute (the unmodified ``release_server.GenerationSession`` and
+``CausalInferencePipeline.inference`` on the drop-ins) is stored in tests/golden/reference_callers_small.npz by
+tests/golden/make_reference_callers_golden.py, which needs the reference checkout.  Each case runs
+tests/run_reference_callers.py in a subprocess (the kernels are swapped for the CPU stand-ins process-wide): the
+harness/ stand-in that bench.py, smoke() and the GPU tests drive must make the same calls and produce the same
+outputs."""
 import json
 import subprocess
 import sys
@@ -10,10 +13,7 @@ from pathlib import Path
 
 import pytest
 
-from tests import ref_env
-
 ROOT = Path(__file__).resolve().parent.parent
-pytestmark = pytest.mark.skipif(not ref_env.available(), reason="reference checkout not present")
 
 
 def run(*args):
@@ -25,10 +25,10 @@ def run(*args):
 
 @pytest.mark.parametrize("mode", ["keep", "reencode"])
 def test_unmodified_generation_session_on_the_dropins(mode):
-    """release_server.py imports cleanly with the finder installed (utils.misc, wan.modules.vae, v2v, settings, ...
-    from the checkout; utils.wan_wrapper / demo_utils.vae_block3 from this repo) and GenerationSession generates 4
-    blocks (window slides at block 2; 'reencode' = the default first-frame re-encode through VAEEncoderWrapper):
-    bit-equal with harness/server_loop.py, within bf16 tolerance of the reference-executed golden."""
+    """release_server.GenerationSession generates 4 blocks on the drop-ins (window slides at block 2; 'reencode' =
+    the default first-frame re-encode through VAEEncoderWrapper): harness/server_loop.py makes the same transformer /
+    VAE calls and reproduces its latents and pixels, and stays within bf16 tolerance of the reference-executed
+    golden."""
     res = run("server", mode)
     assert res["blocks"] == 4 and res["latents_rel_l2"] < 1e-2
 
